@@ -26,9 +26,15 @@ def _entry(rank, world, port, fn, args, errq):
         raise
 
 
-def run_distributed(fn, world, port, args=()):
+def run_distributed(fn, world, port, args=(), cuda=False):
+    """Run ``fn(rank, world, *args)`` on ``world`` spawned ranks.  ``cuda=False``: the ranks see no CUDA device, so they run
+    on CPU over gloo on every machine (with CUDA visible, setup() picks NCCL, which refuses two ranks on one GPU).
+    ``cuda=True``: one GPU per rank, NCCL."""
     ctx = mp.get_context("spawn")
     errq = ctx.SimpleQueue()
+    visible = os.environ.get("CUDA_VISIBLE_DEVICES")
+    if not cuda:
+        os.environ["CUDA_VISIBLE_DEVICES"] = ""        # inherited by the spawned ranks before they load CUDA
     try:
         mp.spawn(_entry, args=(world, port, fn, args, errq), nprocs=world, join=True)
     except Exception as e:
@@ -36,3 +42,8 @@ def run_distributed(fn, world, port, args=()):
         while not errq.empty():
             msgs.append("rank %d:\n%s" % errq.get())
         raise AssertionError("distributed test failed:\n" + "\n".join(msgs) + f"\n{e}")
+    finally:
+        if visible is None:
+            os.environ.pop("CUDA_VISIBLE_DEVICES", None)
+        else:
+            os.environ["CUDA_VISIBLE_DEVICES"] = visible

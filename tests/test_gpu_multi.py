@@ -91,7 +91,7 @@ def _worker_fused(rank, world):
 @need2
 @pytest.mark.parametrize("world", WORLDS)
 def test_fused_tree_attention(world, port):
-    run_distributed(_worker_fused, world, port)
+    run_distributed(_worker_fused, world, port, cuda=True)
 
 
 def _worker_prefill(rank, world):
@@ -150,7 +150,7 @@ def _worker_prefill(rank, world):
 @need2
 @pytest.mark.parametrize("world", WORLDS)
 def test_fused_prefill_tcgen05(world, port):
-    run_distributed(_worker_prefill, world, port)
+    run_distributed(_worker_prefill, world, port, cuda=True)
 
 
 def _worker_zigzag(rank, world):
@@ -204,7 +204,7 @@ def _worker_zigzag(rank, world):
 @need2
 @pytest.mark.parametrize("world", WORLDS)
 def test_zigzag_causal_prefill(world, port):
-    run_distributed(_worker_zigzag, world, port)
+    run_distributed(_worker_zigzag, world, port, cuda=True)
 
 
 def _worker_stress(rank, world):
@@ -233,7 +233,7 @@ def _worker_stress(rank, world):
 
 @need2
 def test_epoch_reuse_stress(port):
-    run_distributed(_worker_stress, 2, port)
+    run_distributed(_worker_stress, 2, port, cuda=True)
 
 
 def _worker_graph(rank, world):
@@ -260,7 +260,7 @@ def _worker_graph(rank, world):
 
 @need2
 def test_fused_cuda_graph_replay(port):
-    run_distributed(_worker_graph, 2, port)
+    run_distributed(_worker_graph, 2, port, cuda=True)
 
 
 def _worker_fault(rank, world):
@@ -287,7 +287,7 @@ def _worker_fault(rank, world):
 
 @need2
 def test_failure_detection_bounded_spin(port):
-    run_distributed(_worker_fault, 2, port)
+    run_distributed(_worker_fault, 2, port, cuda=True)
 
 
 def _worker_reduce_and_bwd(rank, world):
@@ -340,7 +340,7 @@ def _worker_reduce_and_bwd(rank, world):
 
 @need2
 def test_symm_allreduce_and_distributed_backward(port):
-    run_distributed(_worker_reduce_and_bwd, min(NGPU, 4) if NGPU >= 4 else 2, port)
+    run_distributed(_worker_reduce_and_bwd, min(NGPU, 4) if NGPU >= 4 else 2, port, cuda=True)
 
 
 def _worker_fill_levels(rank, world):
@@ -408,4 +408,4 @@ def _worker_fill_levels(rank, world):
 @need2
 @pytest.mark.parametrize("world", WORLDS)
 def test_fused_decode_ragged_fill_levels(world, port):
-    run_distributed(_worker_fill_levels, world, port)
+    run_distributed(_worker_fill_levels, world, port, cuda=True)
